@@ -2,6 +2,7 @@
 """bench.py — rendered Mpix/s (forward+backward, RGB + depth + normal) of the dn-splatter hot path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
+    python bench.py ... --dump-outputs DIR                         # + the last timed step's results as DIR/*.npy
     python bench.py --impl reference ...                           # the reference's CPU path (oracle port)
     torchrun --nproc-per-node N ... bench.py --gpus N ...          # one rank per GPU, per-camera sharding
 
@@ -60,9 +61,41 @@ def parse():
     ap.add_argument("--no-fused-loss-bwd", action="store_true", help="loss gradients as images from separate kernels (A/B)")
     ap.add_argument("--nccl-allreduce", action="store_true", help="multi-rank: dense NCCL all-reduce of the bucket + Adam instead "
                                                                   "of the peer-memory reduction fused into the Adam pass")
-    ap.add_argument("--epochs", type=int, default=5, help="extra, untimed-by-contract measurement: median ms/view over this "
-                                                          "many passes over ALL views (0 = skip)")
-    return ap.parse_args()
+    ap.add_argument("--epochs", type=int, default=0, help="extra measurement after the --steps timed steps: median ms/view "
+                                                          "over this many passes over ALL views (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step produced (loss, per-parameter gradients, "
+                         "parameters after the Adam step; a fixed seeded sample of the Gaussians) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_BYTES = 64_000_000  # the whole --dump-outputs set stays below this
+
+
+def dump_outputs(out_dir, model, bucket, loss):
+    """Writes the results of the last training step as float32 .npy files: `loss`, and for every optimised parameter
+    `<name>` (its value after the optimizer step) and `grad_<name>` (this rank's gradient of the step).  Both are
+    restricted to the same rows: all Gaussians if they fit in DUMP_BYTES, else a sorted sample drawn with a fixed seed,
+    so the rows depend only on the Gaussian count."""
+    import numpy as np
+
+    params = {n: model.gauss_params[n].detach() for n in bucket.names}
+    n = next(iter(params.values())).shape[0]
+    row_bytes = 2 * 4 * sum(p[0].numel() for p in params.values())
+    rows = min(n, (DUMP_BYTES - 65536) // row_bytes)  # 64 KB for the loss and the .npy headers
+    idx = torch.arange(n) if rows == n else torch.randperm(n, generator=torch.Generator().manual_seed(0))[:rows].sort().values
+    idx = idx.to(params[bucket.names[0]].device)
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss.detach().float().reshape(1)}
+    for name, p in params.items():
+        arrays[name] = p.index_select(0, idx)
+        arrays[f"grad_{name}"] = bucket.views[name].index_select(0, idx)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.float().cpu().numpy())
+    return rows
 
 
 # ------------------------------------------------------------------------------------------------ clocks
@@ -391,14 +424,16 @@ def main():
         if optimizer is not None:
             optimizer.step()
 
+    last = {}  # the loss of the latest resident step (for --dump-outputs); detached, so no autograd graph outlives its step
+
     def resident_step(s):
         cam = cams[view_of(s, my_views)]
         if graphed is None:
-            run_step(model, bucket, cam, dev_sets[s % len(dev_sets)], optimizer=optimizer)
+            last["loss"] = run_step(model, bucket, cam, dev_sets[s % len(dev_sets)], optimizer=optimizer).detach()
         else:  # supervision maps: device-resident set -> the graph's static buffers (D2D), then ONE graph launch
             for k, v in dev_sets[s % len(dev_sets)].items():
                 graphed.batches[0][k].copy_(v, non_blocking=True)
-            graphed(cam, 0)
+            last["loss"] = graphed(cam, 0)
             finish_step()
 
     losses = []
@@ -491,6 +526,9 @@ def main():
     if launches_per_step is not None:  # graph replays re-issue the launches recorded at capture (+ the eager Adam step)
         launches = {k: v * args.steps + launches[k] for k, v in launches_per_step.items()}
     clocks = sampler.stop() if rank == 0 else None
+    dumped_rows = None
+    if args.dump_outputs and rank == 0:  # before anything else runs a step: the e2e / epoch passes below train further
+        dumped_rows = dump_outputs(args.dump_outputs, model, bucket, last["loss"])
     pix = args.width * args.height
     value = world * args.steps * pix / 1e6 / (ms / 1e3)
 
@@ -509,7 +547,8 @@ def main():
         e2e = {"value": world * args.steps * pix / 1e6 / (ms_e / 1e3), "unit": "Mpix/s", "h2d_bytes_per_step": h2d_bytes,
                "d2h_bytes_per_step": 4, "ms_per_step": ms_e / args.steps}
 
-    # SURVEY §8d: median over >= 5 passes over the whole view set (the contract's K timed steps above stay the headline)
+    # --epochs E (SURVEY §8d asks for >= 5): median over E passes over the whole view set; the K timed steps above stay
+    # the headline
     epochs = None
     if args.epochs > 0:
         per_epoch = []
@@ -591,6 +630,8 @@ def main():
             "roofline": roof, "stages_ms": stages, "epochs": epochs, "cpu_baseline": cpu, "last_loss": losses[-1] if losses else None,
             "cuda_graph": graph_info, "isect_capacity_report": {str(k): v for k, v in R.capacity_report().items()},
         }
+        if dumped_rows is not None:
+            line["dump_outputs"] = {"dir": args.dump_outputs, "step": args.steps - 1, "gaussian_rows": dumped_rows}
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -1,6 +1,7 @@
 """Generates tests/golden/dn_config_specs.json: what the REFERENCE's dn_config.py (/root/reference/dn_splatter/dn_config.py)
 passes to nerfstudio for its three methods, recorded by executing that file unmodified against stand-in classes that only
-remember their constructor arguments.
+remember their constructor arguments; and tests/golden/dn_model_config_fields.json: every field of the reference's
+DNSplatterModelConfig (dn_splatter/dn_model.py) with the source of its default, in declaration order.
 
     python tests/golden/make_golden_config.py
 """
@@ -53,6 +54,15 @@ REFERENCE_SIDE = {
 }
 
 
+def model_config_fields():
+    """{field name: default expression as source} of the reference's DNSplatterModelConfig class body."""
+    import ast
+
+    tree = ast.parse(open(os.path.join(REF, "dn_splatter", "dn_model.py")).read())
+    cls = next(n for n in tree.body if isinstance(n, ast.ClassDef) and n.name == "DNSplatterModelConfig")
+    return {n.target.id: ast.unparse(n.value) for n in cls.body if isinstance(n, ast.AnnAssign)}
+
+
 def main():
     recording_modules({**NERFSTUDIO, **REFERENCE_SIDE})
     ns = {"__name__": "dn_splatter.dn_config"}
@@ -61,6 +71,11 @@ def main():
     with open(os.path.join(OUT, "dn_config_specs.json"), "w") as f:
         json.dump(specs, f, indent=1, sort_keys=True)
     print(sorted(specs))
+    fields = model_config_fields()
+    with open(os.path.join(OUT, "dn_model_config_fields.json"), "w") as f:
+        json.dump(fields, f, indent=1)
+        f.write("\n")
+    print(list(fields))
 
 
 if __name__ == "__main__":

@@ -66,14 +66,15 @@ def test_method_specifications_match_the_reference(fake_nerfstudio, golden_dir):
         C.no_such_method
 
 
-def test_config_keeps_the_reference_field_names():
+def test_config_keeps_the_reference_field_names(golden_dir):
     """Every field of the reference's DNSplatterModelConfig exists here with the same default (SURVEY §8b, a14)."""
-    import re
+    import ast
 
     from dn_splatter_b200.dn_model import CameraOptimizerConfig, DNSplatterModelConfig
 
     cfg = DNSplatterModelConfig()
-    ref = "/root/reference/dn_splatter/dn_model.py"
+    # every `name: type = default` of the reference's config class, recorded by tests/golden/make_golden_config.py
+    ref = json.load(open(os.path.join(golden_dir, "dn_model_config_fields.json")))
     expect = {"regularization_strategy": "dn-splatter", "use_depth_loss": False, "depth_tolerance": 0.1, "depth_lambda": 0.0,
               "use_depth_smooth_loss": False, "smooth_loss_lambda": 0.1, "predict_normals": True, "use_normal_loss": True,
               "use_normal_cosine_loss": False, "use_normal_tv_loss": True, "normal_supervision": "mono", "normal_lambda": 0.1,
@@ -81,12 +82,11 @@ def test_config_keeps_the_reference_field_names():
               "binary_opacities_threshold": 0.9, "two_d_gaussians": True, "warmup_length": 500, "num_downscales": 0,
               "use_scale_regularization": False, "max_gauss_ratio": 5.0, "stop_split_at": 15000,
               "output_depth_during_training": True, "pearson_lambda": 0}
-    if os.path.exists(ref):  # in the build container: every `name: type = default` line of the reference's config class
-        src = open(ref).read()
-        body = src[src.index("class DNSplatterModelConfig"):src.index("class DNSplatterModel(")]
-        names = set(re.findall(r"^    (\w+): ", body, flags=re.M)) - {"_target"}
-        assert names == set(expect) | {"depth_loss_type", "smooth_loss_type", "camera_optimizer"}
+    assert set(ref) - {"_target"} == set(expect) | {"depth_loss_type", "smooth_loss_type", "camera_optimizer"}
     for k, v in expect.items():
+        assert ast.literal_eval(ref[k]) == v, k
         assert getattr(cfg, k) == v, k
+    assert ref["depth_loss_type"] == "DepthLossType.EdgeAwareLogL1" and ref["smooth_loss_type"] == "DepthLossType.TV"
+    assert "CameraOptimizerConfig(mode='off')" in ref["camera_optimizer"]
     assert isinstance(cfg.camera_optimizer, CameraOptimizerConfig) and cfg.camera_optimizer.mode == "off"
     assert cfg.depth_loss_type.value == "EdgeAwareLogL1" and cfg.smooth_loss_type.value == "TV"
