@@ -70,6 +70,21 @@ class DnrKnnGrid(C.Structure):
     _fields_ = [("lo", _f * 3), ("cell", _f), ("inv_cell", _f), ("dims", C.c_int32 * 3)]
 
 
+class DnrTsdfVolume(C.Structure):
+    """Mirror of struct DnrTsdfVolume (include/dnr.h)."""
+
+    _fields_ = [("voxel_size", C.c_double), ("sdf_trunc", C.c_double), ("depth_trunc", _f), ("capacity", _i),
+                ("hash_size", _i), ("reserved", _i), ("hash_keys", _p), ("hash_vals", _p), ("hash_stamp", _p),
+                ("voxels", _p), ("touched", _p), ("counters", _p)]
+
+
+class DnrTsdfView(C.Structure):
+    """Mirror of struct DnrTsdfView (include/dnr.h)."""
+
+    _fields_ = [("width", _i), ("height", _i), ("stamp", _i), ("reserved", _i), ("fx", _f), ("fy", _f), ("cx", _f), ("cy", _f),
+                ("extrinsic", _f * 16), ("pose", C.c_double * 16), ("depth", _p), ("rgb", _p), ("mask", _p)]
+
+
 POINTER_FIELDS = {n for n, t in DnrArgs._fields_ if t is _p}
 
 _lib: Optional[C.CDLL] = None
@@ -82,6 +97,8 @@ KERNELS_PER_CALL = {
     "dnr_l1_fwd": (1, 0), "dnr_l1_bwd": (1, 0), "dnr_u8_to_f32": (1, 0),
     "dnr_ssim_fwd": (1, 0), "dnr_ssim_bwd": (1, 0), "dnr_ssim_fwd_ex": (1, 0), "dnr_ssim_bwd_ex": (1, 0), "dnr_photometric_fwd": (2, 0), "dnr_photometric_bwd": (1, 0), "dnr_adam_step": (1, 0), "dnr_adam_step_reduce": (2, 0),
     "dnr_knn_build": (2, 1), "dnr_knn_query": (1, 0), "dnr_density": (1, 0), "dnr_ray_densities": (1, 0),
+    "dnr_tsdf_allocate": (1, 0), "dnr_tsdf_integrate": (1, 0), "dnr_tsdf_extract_count": (5, 3), "dnr_tsdf_extract_emit": (1, 0),
+    "dnr_mesh_cluster_count": (8, 4), "dnr_mesh_cluster_emit": (1, 0),
 }
 LAUNCHES = {"handwritten": 0, "cub": 0}
 
@@ -195,6 +212,25 @@ def load():
     lib.dnr_bin_scan_workspace_bytes.argtypes = [C.c_int32]
     lib.dnr_bin_sort_workspace_bytes.restype = C.c_size_t
     lib.dnr_bin_sort_workspace_bytes.argtypes = [C.c_int32, C.c_int64, C.c_int32]
+    V, W = C.POINTER(DnrTsdfVolume), C.POINTER(DnrTsdfView)
+    lib.dnr_tsdf_reset.restype = C.c_int
+    lib.dnr_tsdf_reset.argtypes = [V, C.c_void_p]
+    for name in ("dnr_tsdf_allocate", "dnr_tsdf_integrate"):
+        getattr(lib, name).restype = C.c_int
+        getattr(lib, name).argtypes = [V, W, C.c_void_p]
+    lib.dnr_tsdf_extract_workspace_bytes.restype = C.c_int64
+    lib.dnr_tsdf_extract_workspace_bytes.argtypes = [C.c_int32]
+    lib.dnr_tsdf_extract_count.restype = C.c_int
+    lib.dnr_tsdf_extract_count.argtypes = [V, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p]
+    lib.dnr_tsdf_extract_emit.restype = C.c_int
+    lib.dnr_tsdf_extract_emit.argtypes = [V, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.dnr_mesh_cluster_workspace_bytes.restype = C.c_int64
+    lib.dnr_mesh_cluster_workspace_bytes.argtypes = [C.c_int32, C.c_int32]
+    lib.dnr_mesh_cluster_count.restype = C.c_int
+    lib.dnr_mesh_cluster_count.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p]
+    lib.dnr_mesh_cluster_emit.restype = C.c_int
+    lib.dnr_mesh_cluster_emit.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int64,
+                                          C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     _lib = _Counting(lib)
     return _lib
 
@@ -204,7 +240,9 @@ EXPORTS = (
     "dnr_bin_sort_workspace_bytes", "dnr_bin_sort", "dnr_depth_order_ptr", "dnr_raster_fwd", "dnr_finalize_fwd", "dnr_normal_from_depth",
     "dnr_raster_bwd", "dnr_project_bwd", "dnr_loss_fwd", "dnr_loss_bwd", "dnr_scale_loss_fwd", "dnr_scale_loss_bwd",
     "dnr_l1_fwd", "dnr_l1_bwd", "dnr_u8_to_f32", "dnr_ssim_fwd", "dnr_ssim_bwd", "dnr_ssim_fwd_ex", "dnr_ssim_bwd_ex", "dnr_photometric_fwd", "dnr_photometric_bwd", "dnr_adam_step", "dnr_adam_step_reduce", "dnr_knn_workspace_bytes", "dnr_knn_build", "dnr_knn_query",
-    "dnr_density", "dnr_ray_densities",
+    "dnr_density", "dnr_ray_densities", "dnr_tsdf_reset", "dnr_tsdf_allocate", "dnr_tsdf_integrate",
+    "dnr_tsdf_extract_workspace_bytes", "dnr_tsdf_extract_count", "dnr_tsdf_extract_emit", "dnr_mesh_cluster_workspace_bytes",
+    "dnr_mesh_cluster_count", "dnr_mesh_cluster_emit",
 )
 
 

@@ -27,6 +27,7 @@ SOURCES = {
     "adam.cu": ["-fmad=false"],
     "knn.cu": ["-fmad=false"],
     "density.cu": ["-fmad=false"],
+    "tsdf.cu": ["-fmad=false"],
 }
 
 
@@ -47,7 +48,7 @@ def _stale(target: str, deps) -> bool:
 def build(force: bool = False, verbose: bool = False) -> str:
     nvcc = nvcc_path()
     os.makedirs(OBJ, exist_ok=True)
-    headers = [os.path.join(CSRC, "common.cuh"), os.path.join(CSRC, "loss_common.cuh"), os.path.join(HERE, "..", "include", "dnr.h"), os.path.abspath(__file__)]
+    headers = [os.path.join(CSRC, "common.cuh"), os.path.join(CSRC, "loss_common.cuh"), os.path.join(CSRC, "mc_tables.cuh"), os.path.join(HERE, "..", "include", "dnr.h"), os.path.abspath(__file__)]
     objs = []
     for src, extra in SOURCES.items():
         s = os.path.join(CSRC, src)

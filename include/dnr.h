@@ -318,6 +318,58 @@ int dnr_ray_densities(const float* points, int64_t n_points, const int64_t* nbr_
                       int32_t n_gauss, int32_t n_range, float range_size, float* out_dens, float* out_t, float* out_dirs,
                       void* stream);
 
+/* ---- TSDF mesh extraction (gs-mesh o3dtsdf, export_mesh.py:931-1047; Python surface: dn_splatter_b200.export_mesh) ----
+ * Open3D's legacy ScalableTSDFVolume on the device: volume units of 16^3 voxels in an open-addressing hash, allocated
+ * from the stride-4 depth point cloud and integrated per view; marching cubes over the allocated units; the connected-
+ * cluster filter of the exporter.  Unit coordinates must lie in [-2^20, 2^20) (counters[3] counts points outside). */
+typedef struct DnrTsdfVolume {
+  double voxel_size;   /* voxel edge (Open3D voxel_length) */
+  double sdf_trunc;    /* truncation distance */
+  float depth_trunc;   /* depth > depth_trunc is treated as no depth */
+  int32_t capacity;    /* volume units in the pool */
+  int32_t hash_size;   /* hash slots: a power of two >= capacity */
+  int32_t reserved;
+  void* hash_keys;     /* uint64[hash_size]: packed unit coordinates, ~0 = empty */
+  void* hash_vals;     /* int32[hash_size]: pool slot of the unit, -1 when the pool was full */
+  void* hash_stamp;    /* int32[hash_size]: stamp of the last view that touched the unit */
+  void* voxels;        /* float[capacity][5][4096]: tsdf, weight, r, g, b (0..255); voxel x + 16 y + 256 z */
+  void* touched;       /* int32[hash_size]: hash slots touched by the current view */
+  void* counters;      /* int32[4]: units requested (> capacity = overflow), touched this view, hash full, out of range */
+} DnrTsdfVolume;
+typedef struct DnrTsdfView {
+  int32_t width, height;
+  int32_t stamp;        /* distinct per view since the last reset, >= 0 */
+  int32_t reserved;
+  float fx, fy, cx, cy;
+  float extrinsic[16];  /* world -> camera (OpenCV), fp32, row-major */
+  double pose[16];      /* camera -> world, fp64 (inverse of extrinsic), row-major */
+  const float* depth;   /* [H,W] */
+  const float* rgb;     /* [H,W,3] in [0,1]; the colour used is (uint8)(rgb * 255) */
+  const uint8_t* mask;  /* [H,W] or NULL: 0 = no depth */
+} DnrTsdfView;
+/* Empties the hash, zeroes the pool and the counters. */
+int dnr_tsdf_reset(const DnrTsdfVolume* vol /* HOST struct */, void* stream);
+/* Allocation: inserts the units within sdf_trunc of every stride-4 depth point, lists this view's units. */
+int dnr_tsdf_allocate(const DnrTsdfVolume* vol, const DnrTsdfView* view /* HOST structs */, void* stream);
+/* Integration of the units listed by the last dnr_tsdf_allocate (one CTA per unit, one thread per voxel column). */
+int dnr_tsdf_integrate(const DnrTsdfVolume* vol, const DnrTsdfView* view, void* stream);
+/* Marching cubes over n_units = counters[0] (no overflow) units, in sorted unit order.  extract_count writes int64
+ * {n_vertices, n_triangles} at the start of ws; extract_emit fills vertices / colours [n_vertices,3] f32 and triangles
+ * [n_triangles,3] int32. */
+int64_t dnr_tsdf_extract_workspace_bytes(int32_t n_units);
+int dnr_tsdf_extract_count(const DnrTsdfVolume* vol, int32_t n_units, void* ws, int64_t ws_bytes, void* stream);
+int dnr_tsdf_extract_emit(const DnrTsdfVolume* vol, int32_t n_units, void* ws, int64_t ws_bytes, float* vertices,
+                          float* colors, int32_t* triangles, void* stream);
+/* Cluster filter: triangles sharing an edge are connected; triangles of clusters smaller than
+ * max(size of the keep_largest-th largest cluster (0 if fewer), min_triangles) are removed, then unreferenced vertices;
+ * order is kept.  cluster_count writes int64 {kept vertices, kept triangles} at the start of ws. */
+int64_t dnr_mesh_cluster_workspace_bytes(int32_t n_triangles, int32_t n_vertices);
+int dnr_mesh_cluster_count(const int32_t* triangles, int32_t n_triangles, int32_t n_vertices, int32_t keep_largest,
+                           int32_t min_triangles, void* ws, int64_t ws_bytes, void* stream);
+int dnr_mesh_cluster_emit(const int32_t* triangles, const float* vertices, const float* colors, int32_t n_triangles,
+                          int32_t n_vertices, void* ws, int64_t ws_bytes, int32_t* out_triangles, float* out_vertices,
+                          float* out_colors, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
